@@ -18,6 +18,14 @@ every rank parses its own shard of the stream; record boundaries are shard bound
             the reference cannot be built here (no Go toolchain), so the CPU arm is the
             oracle port (C restatement; AVX-512BW mask routines when the host has them, else AVX2+PCLMUL) run
             ParseNDStream-style on all host threads (10 MiB newline-aligned chunks)
+
+--dump-outputs DIR writes what the last timed step of `value` left in HBM, i.e. what a caller of sj_parse_device
+receives, so that two builds can be compared output for output on the same (deterministic) batch:
+  tape.npy      float64 [k, 2]: high and low 32-bit halves of k tape words (exact in float64)
+  strings.npy   float32 [k]: k bytes of the string buffer
+  sizes.npy     float64 [2]: tape words, string bytes
+k = min(length, 2^21 / ranks); when the output is longer, one position per equal stratum at a seeded offset (a
+fixed sample for a given length).  With N > 1 every rank writes its slice as <name>_rank<r>.npy.  40 MiB of data at most.
 """
 import argparse
 import ctypes as C
@@ -27,6 +35,8 @@ import subprocess
 import sys
 import threading
 import time
+
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as build() left it (it may be read-only)
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
@@ -212,6 +222,32 @@ def k1_traffic(batch_bytes):
         return None
 
 
+DUMP_SAMPLES = 1 << 21
+
+
+def sample_index(length, k, seed):
+    """k increasing positions in [0, length): every position when length <= k, else one per stratum of
+    length // k or more positions, at a seeded offset inside it"""
+    if length <= k:
+        return np.arange(length, dtype=np.int64)
+    rng = np.random.default_rng(seed)
+    return np.arange(k, dtype=np.int64) * length // k + rng.integers(0, length // k, k)
+
+
+def dump_outputs(out_dir, suffix, k, d_tape, tape_words, d_strings, string_bytes):
+    """--dump-outputs: a fixed sample of the tape and string buffer in device memory (see the module docstring)"""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    ti = torch.from_numpy(sample_index(tape_words, k, 1)).to(d_tape.device)
+    words = d_tape[ti].cpu().numpy().view(np.uint64)
+    si = torch.from_numpy(sample_index(string_bytes, k, 2)).to(d_strings.device)
+    sbytes = d_strings[si].cpu().numpy()
+    halves = np.stack([words >> np.uint64(32), words & np.uint64(0xFFFFFFFF)], axis=1)
+    np.save(os.path.join(out_dir, "tape%s.npy" % suffix), halves.astype(np.float64))
+    np.save(os.path.join(out_dir, "strings%s.npy" % suffix), sbytes.astype(np.float32))
+    np.save(os.path.join(out_dir, "sizes%s.npy" % suffix), np.array([tape_words, string_bytes], dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -227,6 +263,7 @@ def main():
     ap.add_argument("--stream-chunk-mib", type=int, default=256, help="chunk size of the library's stream pipeline")
     ap.add_argument("--nccl-exchange", action="store_true", help="N > 1: exchange the shard totals through NCCL even where the peer-memory kernel is available (A/B)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs under ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed sample of the last timed step's tape and strings to DIR/*.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
@@ -355,6 +392,9 @@ def main():
         assert b_host[1] == rank * tape_words and first == b_host[1] + (int(tape_h[0]) & ((1 << 56) - 1)), (b_host, first)
         if exchange == "nccl":
             L.sj_ctx_set_stream(ctx.h, None)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "_rank%d" % rank if world > 1 else "", DUMP_SAMPLES // world,
+                     d_tape, tape_words, d_strings, string_bytes)
 
     # ---- roofline: stage1_flatten alone on the same batch ----
     info = sj.Stage1Info()
